@@ -4,6 +4,7 @@ window frames + <= 10 Gauss-Newton/dogleg iterations of stage C + stage D margin
 HDL-64 sweeps + IMU, window 10/10 (BASELINE.json configs[2], the configuration the metric is quoted on).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload hdl64|vlp16|stress128]
+                  [--dump-outputs DIR]
 
 One "step" = one scan through the whole path.  `value` times the path with the raw sweep already resident
 in HBM; `e2e` times the same call chain through the C-ABI with HOST buffers (pinned host -> device copy of the
@@ -127,8 +128,24 @@ def run_reference(args, scn, W, est_cfg):
             sm = eo.summary()
             iters.append(sm["iterations"]); solve_t.append(sm["t_solve"])
     total = float(np.sum(times))
+    outputs = dict({name: r[key] for name, key in FEATURE_CLOUDS.items()}, states=states[k])
     return dict(scans_per_s=len(times) / total, ms_per_step=1e3 * total / len(times),
-                gn_iter_ms=1e3 * float(np.sum(solve_t)) / max(1.0, float(np.sum(iters))), steps=len(times), states=states)
+                gn_iter_ms=1e3 * float(np.sum(solve_t)) / max(1.0, float(np.sum(iters))), steps=len(times), states=states,
+                outputs=outputs)
+
+
+# stage-A feature clouds of a scan: PointProcessor cloud name -> oracle stage_a key
+FEATURE_CLOUDS = {"corner_points_sharp": "sharp", "corner_points_less_sharp": "less_sharp", "surface_points_flat": "flat",
+                  "surface_points_less_flat": "less_flat"}
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes each array of `outputs` as out_dir/<name>.npy.  Both arms write the same names (the window states and the
+    stage-A feature clouds of the last timed scan), so that two builds, or a build and the oracle, compare file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def host_cores():
@@ -162,7 +179,12 @@ def main():
                     help="multi-GPU: peer = per-scan exchange of the features over peer memory (default); rows = S blocks stored from the "
                          "stage-C kernel tail at every evaluation; nccl = allreduce callback of the S blocks")
     ap.add_argument("--cpu-sample", type=int, default=4, help="scans of the cpu_baseline sample (rank 0, N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed scan returned as DIR/<name>.npy: the window states "
+                         "(float64, window+1 x 16) and the four stage-A feature clouds (float32, n x 4); a few MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
 
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
@@ -180,6 +202,8 @@ def main():
             return 0
         scn = scenario.Scenario(kind, n_total=n_total)
         r = run_reference(args, scn, W, est_cfg)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, r["outputs"])
         cores = 4   # threads the restatement actually uses: 1 (front end, kNN, dogleg: Ceres num_threads = 1) + 4 only inside ThreadsConstructA
         line = {"impl": "reference", "metric": METRIC, "value": r["scans_per_s"], "unit": "scans/s", "n_gpus": args.gpus,
                 "steps": args.steps, "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True,
@@ -352,6 +376,8 @@ def main():
         total_ms = float(t.item())
     prof = est.kernel_profile()
     final_states = est.states()
+    if args.dump_outputs and rank == 0:    # before the e2e pass reuses the point processor
+        dump_outputs(args.dump_outputs, dict({name: pp.cloud(name) for name in FEATURE_CLOUDS}, states=final_states))
 
     if profiling:
         print(json.dumps({"profiling_run": True, "ms_per_step_under_profiler": total_ms / args.steps}))
