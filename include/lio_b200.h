@@ -147,7 +147,9 @@ int lio_laser_odom_host(const float *map, int K, const float *surf, int M, float
  * num_stack_frames_ == 1): associate the odometry increment (:753-756), bring the last features to the map frame and back
  * (:782-800, :1013-1016), re-centre the cube array (:809-931), select the cubes in the field of view (:944-1003), pull
  * laser_cloud_{corner,surf}_from_map_ (:1005-1011), VoxelGrid the stacks (:1016-1022), OptimizeTransformTobeMapped
- * (:325-753) and UpdateMapDatabase (:1112-1208: order-preserving insert + VoxelGrid of every valid cube).
+ * (:325-753) and UpdateMapDatabase (:1112-1208: order-preserving insert + VoxelGrid of every valid cube).  The insert runs
+ * on the device (stable sort by cube, scatter to the append positions); the host only grows segments from the per-cube add
+ * counts.  The per-cube VoxelGrid workspace grows with the largest cube, so a cube above max_points is no error.
  * transform_sum7 = transform_sum_ from the odometry (qx qy qz qw px py pz); out: transform_tobe_mapped_ and
  * info3 = {iterations, corner_from_map size, surf_from_map size}.  Cube index = i + 21 j + 441 k (PointMapping.h:150-153). */
 typedef struct lio_pm lio_pm;
@@ -189,6 +191,34 @@ int lio_po_cloud_download(lio_po *po, int which, float *out_xyzi, int cap);
 int lio_po_compact_data(lio_po *po, float *out_xyzi, int cap_points, int *n_points);
 int lio_po_last_launches(lio_po *po);
 int lio_po_matches(lio_po *po, int kind, int32_t *out, int cap_queries);   /* test aid: indices of the last search, 2 (corner) / 3 (surf) per query */
+
+/* ---- The pre-initialisation chain on the device: stage A -> PointOdometry -> PointMapping without host copies ------------
+ * (the reference's processor -> odometry -> mapping node graph; Estimator::ProcessCompactData runs PointMapping::Process
+ * before IMU initialisation, Estimator.cc:776-848).  Semantics and outputs equal the _host entries; errors follow them.
+ * Streams: the entries enqueue on the context's own stream.  The caller orders them after the producer, by sharing one
+ * stream or by recording an event, exactly as with lio_est_process_scan_dev.
+ * Lifetime of inputs: the input clouds are only read during the call (each call ends with its read-back).  The odometry
+ * context copies into its own buffers whatever must outlive the call - the less-sharp / less-flat clouds that become the
+ * "last" clouds and the full cloud of the payload - so the producer (lio_pp) may process the next sweep right away. */
+/* A cloud on the device whose point count lives in device memory (e.g. lio_pp_cloud_dev + lio_pp_cloud_count_dev).
+ * The count is read on the device and clamped there to n_max; n_max above the context's capacity is LIO_ERR_CAPACITY
+ * before anything is enqueued.  n_max == 0 stands for an empty cloud (xyzi / n_dev may then be NULL). */
+typedef struct lio_dev_cloud { const float *xyzi; const int *n_dev; int n_max; } lio_dev_cloud;
+
+/* PointOdometry::Process + PublishResults on device clouds, in the order sharp, less_sharp, flat, less_flat, full.
+ * At most one host synchronisation: the final read-back of transform_es_, the iteration / match counts and the five counts. */
+int lio_po_process_dev(lio_po *po, const lio_dev_cloud clouds[5], float transform_sum7[7], float transform_es7[7], int info4[4]);
+/* last_corner_cloud_ / last_surf_cloud_ / full_cloud_ (which 0/1/2) with a device count; valid until the next lio_po_process_*. */
+int lio_po_cloud_dev(lio_po *po, int which, const float **xyzi, const int **n_dev);
+/* PointMapping::Process on device clouds (e.g. lio_po_cloud_dev 0 and 1); transform_sum7 on the host as lio_po_process_* returns it.
+ * At most 4 host synchronisations in a call that grows no workspace (growing a cube segment is stream-ordered and costs none;
+ * re-allocating the scan-to-map or re-filter workspace adds one). */
+int lio_pm_process_dev(lio_pm *pm, const lio_dev_cloud *corner_last, const lio_dev_cloud *surf_last, const float transform_sum7[7],
+                       float transform_tobe_mapped7[7], int info3[3]);
+/* What the last process call cost the host: {kernel launches, host synchronisations (stream synchronisations and the device
+ * synchronisation of a workspace re-allocation), bytes host->device, bytes device->host}. */
+int lio_po_last_stats(lio_po *po, long long out[4]);
+int lio_pm_last_stats(lio_pm *pm, long long out[4]);
 
 /* PointMapping::OptimizeTransformTobeMapped (PointMapping.cc:325-753): scan-to-map 6-DoF float Gauss-Newton of
  * transform_tobe_mapped_ (tf7, in/out) against explicit corner / surf maps (laser_cloud_corner_from_map_ /

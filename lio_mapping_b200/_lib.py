@@ -41,6 +41,11 @@ class EstConfig(C.Structure):
                 ("device_solver", C.c_int), ("overlap_marginalization", C.c_int), ("solver_graph", C.c_int)]
 
 
+class DevCloud(C.Structure):
+    """lio_dev_cloud (include/lio_b200.h): a device cloud whose point count lives in device memory, bounded by n_max."""
+    _fields_ = [("xyzi", C.c_void_p), ("n_dev", C.c_void_p), ("n_max", C.c_int)]
+
+
 ALLREDUCE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_int)
 
 
@@ -107,6 +112,12 @@ def lib():
     L.lio_po_compact_data.argtypes = [vp, f32p, ip, C.POINTER(ip)]
     L.lio_po_last_launches.argtypes = [vp]
     L.lio_po_matches.argtypes = [vp, ip, i32p, ip]
+    L.lio_po_process_dev.argtypes = [vp, C.POINTER(DevCloud), f32p, f32p, i32p]
+    L.lio_po_cloud_dev.argtypes = [vp, ip, C.POINTER(vp), C.POINTER(vp)]
+    L.lio_pm_process_dev.argtypes = [vp, C.POINTER(DevCloud), C.POINTER(DevCloud), f32p, f32p, i32p]
+    i64p = np.ctypeslib.ndpointer(np.int64, flags="C_CONTIGUOUS")
+    L.lio_po_last_stats.argtypes = [vp, i64p]
+    L.lio_pm_last_stats.argtypes = [vp, i64p]
     L.lio_transform_to_end_host.argtypes = [f32p, ip, f32p, C.c_float, ip]
     L.lio_laser_odom_host.argtypes = [f32p, ip, f32p, ip, f32p, C.c_float, C.c_float, ip, ip, f32p, f32p, i32p,
                                       C.POINTER(ip), C.POINTER(ip), ip]

@@ -20,6 +20,25 @@ namespace lio {
 
 constexpr int kWarp = 32;
 
+// What one process call cost the host (lio_po_last_stats / lio_pm_last_stats): kernel launches, stream synchronisations
+// and the bytes of every host<->device copy the call enqueued.
+struct CallStats {
+  long long launches = 0, syncs = 0, h2d = 0, d2h = 0;
+  void reset() { launches = syncs = h2d = d2h = 0; }
+};
+inline cudaError_t stats_h2d(CallStats &s, void *dst, const void *src, size_t bytes, cudaStream_t st) {
+  s.h2d += (long long)bytes;
+  return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st);
+}
+inline cudaError_t stats_d2h(CallStats &s, void *dst, const void *src, size_t bytes, cudaStream_t st) {
+  s.d2h += (long long)bytes;
+  return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st);
+}
+inline cudaError_t stats_sync(CallStats &s, cudaStream_t st) {
+  ++s.syncs;
+  return cudaStreamSynchronize(st);
+}
+
 __device__ __forceinline__ unsigned lane_id() { return threadIdx.x & 31; }
 __device__ __forceinline__ unsigned warp_id() { return threadIdx.x >> 5; }
 

@@ -8,7 +8,9 @@
 //                                            OptimizeTransformTobeMapped (scan_to_map_run: voxel-hash k-NN + 6 x 6 float GN)
 //   UpdateMapDatabase          :1112-1208    order-preserving insert into the cubes + VoxelGrid of every touched valid cube
 // Per-point work runs in kernels; the 4851-entry cube directory (pointer, count, capacity per cube) lives on the host and is
-// the only thing the control logic touches.  Compiled with -fmad=false: the float expressions follow the reference's order,
+// the only thing the control logic touches.  The insert is a stable radix sort of (cube, input index) followed by a scatter
+// to `append position of the cube + rank in its run`; the host reads only the per-cube add counts, grows the segments and
+// uploads the append positions of the touched cubes (the device mirror of the directory the scatter reads).  Compiled with -fmad=false: the float expressions follow the reference's order,
 // clouds, cube contents and the mapped pose are compared with the oracle (oracle/o_cubemap.cc).
 #include <algorithm>
 #include <cmath>
@@ -41,21 +43,24 @@ __device__ __forceinline__ void rotate_dev(float qx, float qy, float qz, float q
   ox = vx + ux * qw + cx; oy = vy + uy * qw + cy; oz = vz + uz * qw + cz;
 }
 
-// mode 0: PointAssociateToMap (po = q * pi + t, :303-314); mode 1: PointAssociateTobeMapped (po = q^* * (pi - t), :316-323)
+// PointAssociateToMap (po = q * pi + t, :303-314) followed by PointAssociateTobeMapped (po = q^* * (pi - t), :316-323): the
+// reference stacks the last features in the map frame and takes them back before the VoxelGrid (:782-800, :1013-1016).
+// Both float steps in the reference's order (-fmad=false), the intermediate kept in registers.  The count is read on the
+// device and clamped to n_max; CTA 0 publishes the clamped count in n_out for the kernels after it.
 __global__ void __launch_bounds__(256)
-k_associate(const float4 *__restrict__ in, float4 *__restrict__ out, const int *__restrict__ n_dev, TwistF t, int mode) {
-  const int n = *n_dev;
+k_associate(const float4 *__restrict__ in, float4 *__restrict__ out, const int *__restrict__ n_dev, int n_max, int *__restrict__ n_out, TwistF t) {
+  int n = *n_dev;
+  n = n < 0 ? 0 : (n > n_max ? n_max : n);
+  if (blockIdx.x == 0 && threadIdx.x == 0) *n_out = n;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const float4 p = __ldg(in + i);
   float x, y, z;
-  if (mode == 0) {
-    rotate_dev(t.qx, t.qy, t.qz, t.qw, p.x, p.y, p.z, x, y, z);
-    x += t.px; y += t.py; z += t.pz;
-  } else {
-    rotate_dev(-t.qx, -t.qy, -t.qz, t.qw, p.x - t.px, p.y - t.py, p.z - t.pz, x, y, z);
-  }
-  out[i] = make_float4(x, y, z, p.w);
+  rotate_dev(t.qx, t.qy, t.qz, t.qw, p.x, p.y, p.z, x, y, z);
+  x += t.px; y += t.py; z += t.pz;
+  float bx, by, bz;
+  rotate_dev(-t.qx, -t.qy, -t.qz, t.qw, x - t.px, y - t.py, z - t.pz, bx, by, bz);
+  out[i] = make_float4(bx, by, bz, p.w);
 }
 
 // int((v + 25.0) / 50.0) + cen, minus one for negatives (:812-819) - double arithmetic like the reference
@@ -65,29 +70,49 @@ __device__ __forceinline__ int cube_of(float v, int cen) {
   return c;
 }
 
-// UpdateMapDatabase insert, phase 1: map-frame point and destination cube of every down-sampled stack point (-1: outside)
+constexpr int kKeyStride = 8192;   // sort key = cloud * kKeyStride + cube; kCubes (outside the array) sorts last in its cloud
+constexpr int kKeyBits = 14;
+
+// UpdateMapDatabase insert, phase 1, over both down-sampled stacks (corner: [0, n0), surf: [n0, n0 + n1)): map-frame point,
+// sort key and per-cube add count of every point
 __global__ void __launch_bounds__(256)
-k_cube_ids(const float4 *__restrict__ in, const int *__restrict__ n_dev, TwistF t, int cen_l, int cen_w, int cen_h, float4 *__restrict__ mapped,
-           int *__restrict__ cube) {
-  const int n = *n_dev;
+k_cube_ids(const float4 *__restrict__ ds0, int n0, const float4 *__restrict__ ds1, int n1, TwistF t, int cen_l, int cen_w, int cen_h,
+           float4 *__restrict__ mapped, unsigned *__restrict__ key, unsigned *__restrict__ val, int *__restrict__ add, int *__restrict__ n_tot) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const float4 p = __ldg(in + i);
+  if (i == 0) *n_tot = n0 + n1;
+  if (i >= n0 + n1) return;
+  const int w = i >= n0 ? 1 : 0;
+  const float4 p = w ? __ldg(ds1 + (i - n0)) : __ldg(ds0 + i);
   float x, y, z;
   rotate_dev(t.qx, t.qy, t.qz, t.qw, p.x, p.y, p.z, x, y, z);
   x += t.px; y += t.py; z += t.pz;
   mapped[i] = make_float4(x, y, z, p.w);
   const int ci = cube_of(x, cen_l), cj = cube_of(y, cen_w), ck = cube_of(z, cen_h);
-  cube[i] = (ci >= 0 && ci < kCubeL && cj >= 0 && cj < kCubeW && ck >= 0 && ck < kCubeH) ? ci + kCubeL * cj + kCubeL * kCubeW * ck : -1;
+  const bool inside = ci >= 0 && ci < kCubeL && cj >= 0 && cj < kCubeW && ck >= 0 && ck < kCubeH;
+  const int c = inside ? ci + kCubeL * cj + kCubeL * kCubeW * ck : kCubes;
+  key[i] = (unsigned)(w * kKeyStride + c);
+  val[i] = (unsigned)i;
+  if (inside) atomicAdd(add + w * kCubes + c, 1);
 }
 
-// phase 2: dst[i] is the address the host directory assigned to point i (append position inside its cube, input order kept)
+// phase 2, after the stable sort: the first position of every key's run
+__global__ void __launch_bounds__(256) k_run_heads(const unsigned *__restrict__ key, int n, int *__restrict__ start) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= n) return;
+  const unsigned k = key[s];
+  if (s == 0 || key[s - 1] != k) start[k] = s;
+}
+
+// phase 3: sorted position s goes to the append position of its cube + its rank in the run - the push_back order of the
+// input, because the sort is stable
 __global__ void __launch_bounds__(256)
-k_scatter_to_cubes(const float4 *__restrict__ mapped, float4 *const *__restrict__ dst, int n) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  float4 *d = dst[i];
-  if (d) *d = __ldg(mapped + i);
+k_scatter_to_cubes(const float4 *__restrict__ mapped, const unsigned *__restrict__ key, const unsigned *__restrict__ val, const int *__restrict__ start,
+                   float4 *const *__restrict__ base, int n) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= n) return;
+  const unsigned k = key[s];
+  if ((int)(k % kKeyStride) == kCubes) return;
+  base[k][s - start[k]] = __ldg(mapped + val[s]);
 }
 
 struct Segment { const float4 *src; int n; int off; };
@@ -103,6 +128,17 @@ k_gather_segments(const Segment *__restrict__ seg, int nseg, float4 *__restrict_
 }  // namespace lio
 
 using namespace lio;
+
+// Pinned staging of one process call (written by the host, read by async copies that complete before the call's last
+// synchronisation, or before the first one of the next call).
+struct PmStage {
+  int cnt_up[2];                        // host-path input counts
+  int n_ds[2];                          // read-back: down-sampled stack sizes
+  int add[2 * kCubes];                  // read-back: points each cube receives (corner, surf)
+  float4 *base[2 * kKeyStride];         // append position of every touched cube, by sort key
+  Segment seg[2][256];                  // laser_cloud_{corner,surf}_from_map_ segments
+  int vgn[256], vgout[256];             // re-filter input / output counts
+};
 
 struct lio_pm {
   struct Cube { float4 *p = nullptr; int n = 0, cap = 0; };
@@ -121,9 +157,12 @@ struct lio_pm {
   float4 *d_in[2] = {nullptr, nullptr}, *d_stack[2] = {nullptr, nullptr}, *d_ds[2] = {nullptr, nullptr}, *d_mapped = nullptr, *d_tmp = nullptr;
   float4 *d_map[2] = {nullptr, nullptr};
   int map_cap[2] = {0, 0};
-  int *d_cnt = nullptr;                // [0,1] input sizes, [2,3] down-sampled sizes, [4..] voxel-grid outputs
-  int *d_cube = nullptr;
-  float4 **d_dst = nullptr;
+  int *d_cnt = nullptr;                // [0,1] clamped input sizes, [2,3] down-sampled sizes, [4,5] host-path input sizes, [6] insert size, [7] 0
+  unsigned *d_key[2] = {nullptr, nullptr}, *d_val[2] = {nullptr, nullptr};   // insert sort ping-pong (2 max_points)
+  RadixSortTemp rs;
+  int *d_add = nullptr;                // 2 x kCubes
+  int *d_start = nullptr;              // 2 x kKeyStride run heads
+  float4 **d_base = nullptr;           // 2 x kKeyStride append positions (device mirror of the touched directory entries)
   Segment *d_seg = nullptr;
   int *d_vgout = nullptr;              // per re-filtered cube: output count
   VoxelGrid vg;
@@ -131,8 +170,8 @@ struct lio_pm {
   ScanToMapWork stm;
   int stm_cap[3] = {0, 0, 0};
   int last_iters = 0, last_from_map[2] = {0, 0};
-  std::vector<int> h_cube;
-  std::vector<float4 *> h_dst;
+  PmStage *h = nullptr;
+  CallStats stats;
 };
 
 static size_t to_index(int i, int j, int k) { return (size_t)i + (size_t)kCubeL * j + (size_t)kCubeL * kCubeW * k; }
@@ -147,11 +186,13 @@ extern "C" int lio_pm_destroy(lio_pm *m) {
   cudaSetDevice(m->device);
   for (int w = 0; w < 2; ++w) {
     for (lio_pm::Cube &c : m->cube[w]) if (c.p) cudaFree(c.p);
-    void *fr[] = {m->d_in[w], m->d_stack[w], m->d_ds[w], m->d_map[w]};
+    void *fr[] = {m->d_in[w], m->d_stack[w], m->d_ds[w], m->d_map[w], m->d_key[w], m->d_val[w]};
     for (void *q : fr) if (q) cudaFree(q);
   }
-  void *fr[] = {m->d_mapped, m->d_tmp, m->d_cnt, m->d_cube, m->d_dst, m->d_seg, m->d_vgout};
+  void *fr[] = {m->d_mapped, m->d_tmp, m->d_cnt, m->d_add, m->d_start, m->d_base, m->d_seg, m->d_vgout};
   for (void *q : fr) if (q) cudaFree(q);
+  if (m->h) cudaFreeHost(m->h);
+  m->rs.destroy();
   m->vg.destroy();
   m->stm.destroy();
   delete m;
@@ -176,19 +217,22 @@ extern "C" int lio_pm_create(int max_points, float corner_filter_size, float sur
     ok = ok && cudaMalloc(&m->d_in[w], sizeof(float4) * max_points) == cudaSuccess;
     ok = ok && cudaMalloc(&m->d_stack[w], sizeof(float4) * max_points) == cudaSuccess;
     ok = ok && cudaMalloc(&m->d_ds[w], sizeof(float4) * max_points) == cudaSuccess;
+    ok = ok && cudaMalloc(&m->d_key[w], sizeof(unsigned) * 2 * max_points) == cudaSuccess;
+    ok = ok && cudaMalloc(&m->d_val[w], sizeof(unsigned) * 2 * max_points) == cudaSuccess;
   }
-  ok = ok && cudaMalloc(&m->d_mapped, sizeof(float4) * max_points) == cudaSuccess;
-  ok = ok && cudaMalloc(&m->d_cnt, sizeof(int) * 8) == cudaSuccess;
-  ok = ok && cudaMalloc(&m->d_cube, sizeof(int) * max_points) == cudaSuccess;
-  ok = ok && cudaMalloc(&m->d_dst, sizeof(float4 *) * max_points) == cudaSuccess;
+  ok = ok && cudaMalloc(&m->d_mapped, sizeof(float4) * 2 * max_points) == cudaSuccess;
+  ok = ok && cudaMalloc(&m->d_cnt, sizeof(int) * 8) == cudaSuccess && cudaMemset(m->d_cnt, 0, sizeof(int) * 8) == cudaSuccess;
+  ok = ok && m->rs.init(2 * max_points) == 0;
+  ok = ok && cudaMalloc(&m->d_add, sizeof(int) * 2 * kCubes) == cudaSuccess;
+  ok = ok && cudaMalloc(&m->d_start, sizeof(int) * 2 * kKeyStride) == cudaSuccess;
+  ok = ok && cudaMalloc(&m->d_base, sizeof(float4 *) * 2 * kKeyStride) == cudaSuccess;
   ok = ok && cudaMalloc(&m->d_seg, sizeof(Segment) * 256) == cudaSuccess;
   ok = ok && cudaMalloc(&m->d_vgout, sizeof(int) * 256) == cudaSuccess;
+  ok = ok && cudaMallocHost(&m->h, sizeof(PmStage)) == cudaSuccess;
   m->vg_cap = max_points;
   ok = ok && cudaMalloc(&m->d_tmp, sizeof(float4) * m->vg_cap) == cudaSuccess;
   ok = ok && m->vg.init(m->vg_cap) == 0;
   if (!ok) { lio_set_last_error(__FILE__, __LINE__, "lio_pm_create: device allocation failed"); lio_pm_destroy(m); return LIO_ERR_CUDA; }
-  m->h_cube.resize(max_points);
-  m->h_dst.resize(max_points);
   *out = m;
   return LIO_OK;
 }
@@ -253,121 +297,152 @@ static void pm_select(const lio_pm *m, float px, float py, float pz, const float
       }
 }
 
+// Segments (and the pulled maps) come from the stream-ordered allocator: allocation, copy of the old contents and release of
+// the old segment are all enqueued on the context's stream, so growing a cube costs the host no synchronisation.
 static int pm_grow(lio_pm *m, lio_pm::Cube &c, int need) {
   if (need <= c.cap) return LIO_OK;
   int cap = std::max(1024, c.cap);
   while (cap < need) cap *= 2;
   float4 *p = nullptr;
-  LIO_CUDA_OK(cudaMalloc(&p, sizeof(float4) * cap));
+  LIO_CUDA_OK(cudaMallocAsync((void **)&p, sizeof(float4) * cap, m->stream));
   if (c.p && c.n > 0) LIO_CUDA_OK(cudaMemcpyAsync(p, c.p, sizeof(float4) * c.n, cudaMemcpyDeviceToDevice, m->stream));
-  if (c.p) { LIO_CUDA_OK(cudaStreamSynchronize(m->stream)); cudaFree(c.p); }
+  if (c.p) LIO_CUDA_OK(cudaFreeAsync(c.p, m->stream));
   c.p = p; c.cap = cap;
   return LIO_OK;
 }
 
 // laser_cloud_*_from_map_: concatenate the valid cubes (in `valid` order) into d_map[w]
 static int pm_from_map(lio_pm *m, const std::vector<size_t> &valid, int w, int &total) {
-  std::vector<Segment> seg;
+  Segment *seg = m->h->seg[w];
+  int nseg = 0;
   total = 0;
   for (size_t v : valid) {
     const lio_pm::Cube &c = m->cube[w][v];
-    if (c.n > 0) { seg.push_back(Segment{c.p, c.n, total}); total += c.n; }
+    if (c.n > 0) {
+      if (nseg == 256) return LIO_ERR_CAPACITY;
+      seg[nseg++] = Segment{c.p, c.n, total};
+      total += c.n;
+    }
   }
   if (total > m->map_cap[w]) {
-    if (m->d_map[w]) cudaFree(m->d_map[w]);
+    if (m->d_map[w]) LIO_CUDA_OK(cudaFreeAsync(m->d_map[w], m->stream));
+    m->d_map[w] = nullptr;
     m->map_cap[w] = std::max(2 * total, 1 << 16);
-    LIO_CUDA_OK(cudaMalloc(&m->d_map[w], sizeof(float4) * m->map_cap[w]));
+    LIO_CUDA_OK(cudaMallocAsync((void **)&m->d_map[w], sizeof(float4) * m->map_cap[w], m->stream));
   }
-  if (seg.empty()) return LIO_OK;
-  if (seg.size() > 256) return LIO_ERR_CAPACITY;
-  LIO_CUDA_OK(cudaMemcpyAsync(m->d_seg, seg.data(), sizeof(Segment) * seg.size(), cudaMemcpyHostToDevice, m->stream));
-  LIO_CUDA_OK(cudaStreamSynchronize(m->stream));   // seg is a stack vector
-  k_gather_segments<<<dim3(16, (unsigned)seg.size()), 256, 0, m->stream>>>(m->d_seg, (int)seg.size(), m->d_map[w]);
+  if (nseg == 0) return LIO_OK;
+  LIO_CUDA_OK(stats_h2d(m->stats, m->d_seg, seg, sizeof(Segment) * nseg, m->stream));
+  k_gather_segments<<<dim3(16, (unsigned)nseg), 256, 0, m->stream>>>(m->d_seg, nseg, m->d_map[w]);
+  ++m->stats.launches;
   return LIO_OK;
 }
 
 // UpdateMapDatabase (:1112-1208) with margin centre == current centre (the valid list was computed in this call)
 static int pm_update(lio_pm *m, const std::vector<size_t> &valid, const int n_ds[2]) {
   cudaStream_t st = m->stream;
-  for (int w = 0; w < 2; ++w) {
-    const int n = n_ds[w];
-    if (n == 0) continue;
-    k_cube_ids<<<(n + 255) / 256, 256, 0, st>>>(m->d_ds[w], m->d_cnt + 2 + w, m->tobe, m->cen_l, m->cen_w, m->cen_h, m->d_mapped, m->d_cube);
-    LIO_CUDA_OK(cudaMemcpyAsync(m->h_cube.data(), m->d_cube, sizeof(int) * n, cudaMemcpyDeviceToHost, st));
-    LIO_CUDA_OK(cudaStreamSynchronize(st));
-    // append positions in input order (push_back order): first the per-cube totals to size the segments, then the addresses
-    std::vector<int> add(kCubes, 0);
-    for (int i = 0; i < n; ++i) if (m->h_cube[i] >= 0) ++add[m->h_cube[i]];
-    for (int c = 0; c < kCubes; ++c)
-      if (add[c]) { int rc = pm_grow(m, m->cube[w][c], m->cube[w][c].n + add[c]); if (rc != LIO_OK) return rc; }
-    for (int i = 0; i < n; ++i) {
-      const int c = m->h_cube[i];
-      if (c < 0) { m->h_dst[i] = nullptr; continue; }
-      lio_pm::Cube &cb = m->cube[w][c];
-      m->h_dst[i] = cb.p + cb.n;
-      ++cb.n;
-    }
-    LIO_CUDA_OK(cudaMemcpyAsync(m->d_dst, m->h_dst.data(), sizeof(float4 *) * n, cudaMemcpyHostToDevice, st));
-    k_scatter_to_cubes<<<(n + 255) / 256, 256, 0, st>>>(m->d_mapped, m->d_dst, n);
-    LIO_CUDA_OK(cudaStreamSynchronize(st));   // h_dst is reused by the next cloud
-  }
-  // re-filter every valid cube (corner then surf), each with its own bounding box like pcl::VoxelGrid on that cube's cloud
-  struct Job { int w; size_t idx; };
-  std::vector<Job> jobs;
+  CallStats &S = m->stats;
+  PmStage *h = m->h;
+  // the cubes re-filtered after the insert (corner then surf of every valid cube), each with its own bounding box like
+  // pcl::VoxelGrid on that cube's cloud
+  std::vector<size_t> refilter;
   for (size_t index : valid) {
     int li, lj, lk;
     { int residual = (int)(index % (kCubeL * kCubeW)); lk = (int)(index / (kCubeL * kCubeW)); lj = residual / kCubeL; li = residual % kCubeL; }
     const float center_x = 50.0f * (li - m->cen_l), center_y = 50.0f * (lj - m->cen_w), center_z = 50.0f * (lk - m->cen_h);
     const int ci = cube_of_host(center_x, m->cen_l), cj = cube_of_host(center_y, m->cen_w), ck = cube_of_host(center_z, m->cen_h);
     if (!(ci >= 0 && ci < kCubeL && cj >= 0 && cj < kCubeW && ck >= 0 && ck < kCubeH)) continue;
-    const size_t idx = to_index(ci, cj, ck);
-    for (int w = 0; w < 2; ++w) if (m->cube[w][idx].n > 0) jobs.push_back(Job{w, idx});
+    refilter.push_back(to_index(ci, cj, ck));
   }
+  const int n = n_ds[0] + n_ds[1];
+  if (n > 0) {
+    // insert: cube ids + add counts, stable sort of (cloud, cube | input index), run heads; the add counts come back
+    LIO_CUDA_OK(cudaMemsetAsync(m->d_add, 0, sizeof(int) * 2 * kCubes, st));
+    const int nb = (n + 255) / 256;
+    k_cube_ids<<<nb, 256, 0, st>>>(m->d_ds[0], n_ds[0], m->d_ds[1], n_ds[1], m->tobe, m->cen_l, m->cen_w, m->cen_h, m->d_mapped, m->d_key[0],
+                                   m->d_val[0], m->d_add, m->d_cnt + 6);
+    int launches = 1;
+    const int which = radix_sort_pairs(m->d_key[0], m->d_val[0], m->d_key[1], m->d_val[1], m->d_cnt + 6, n, kKeyBits, m->rs, st, &launches);
+    if (which < 0) { lio_set_last_error(__FILE__, __LINE__, "cube insert: sort workspace too small"); return LIO_ERR_CAPACITY; }
+    const unsigned *skey = m->d_key[which], *sval = m->d_val[which];
+    k_run_heads<<<nb, 256, 0, st>>>(skey, n, m->d_start);
+    ++launches;
+    S.launches += launches;
+    LIO_CUDA_OK(stats_d2h(S, h->add, m->d_add, sizeof(int) * 2 * kCubes, st));
+    LIO_CUDA_OK(stats_sync(S, st));
+    // grow the receiving segments, then the re-filter workspace to the largest cube it will see - before anything moves, so
+    // a failure leaves the map as it was
+    int need_vg = 0;
+    for (int w = 0; w < 2; ++w)
+      for (int c = 0; c < kCubes; ++c)
+        if (h->add[w * kCubes + c]) { int rc = pm_grow(m, m->cube[w][c], m->cube[w][c].n + h->add[w * kCubes + c]); if (rc != LIO_OK) return rc; }
+    for (size_t idx : refilter)
+      for (int w = 0; w < 2; ++w) need_vg = std::max(need_vg, m->cube[w][idx].n + h->add[w * kCubes + idx]);
+    if (need_vg > m->vg_cap) {
+      int cap = m->vg_cap;
+      while (cap < need_vg) cap *= 2;
+      ++S.syncs;   // cudaFree synchronises the device
+      m->vg.destroy();
+      if (m->d_tmp) cudaFree(m->d_tmp);
+      m->d_tmp = nullptr;
+      m->vg_cap = 0;
+      if (cudaMalloc(&m->d_tmp, sizeof(float4) * cap) != cudaSuccess || m->vg.init(cap) != 0) {
+        lio_set_last_error(__FILE__, __LINE__, "cube re-filter workspace allocation failed");
+        return LIO_ERR_CUDA;
+      }
+      m->vg_cap = cap;
+    }
+    // append positions of the touched cubes, one contiguous key range per cloud
+    for (int w = 0; w < 2; ++w) {
+      int lo = kCubes, hi = -1;
+      for (int c = 0; c < kCubes; ++c)
+        if (h->add[w * kCubes + c]) {
+          lo = std::min(lo, c); hi = c;
+          h->base[w * kKeyStride + c] = m->cube[w][c].p + m->cube[w][c].n;
+        }
+      if (hi >= lo) LIO_CUDA_OK(stats_h2d(S, m->d_base + w * kKeyStride + lo, h->base + w * kKeyStride + lo, sizeof(float4 *) * (hi - lo + 1), st));
+    }
+    k_scatter_to_cubes<<<nb, 256, 0, st>>>(m->d_mapped, skey, sval, m->d_start, m->d_base, n);
+    ++S.launches;
+    for (int w = 0; w < 2; ++w)
+      for (int c = 0; c < kCubes; ++c) m->cube[w][c].n += h->add[w * kCubes + c];
+  }
+  struct Job { int w; size_t idx; };
+  std::vector<Job> jobs;
+  for (size_t idx : refilter)
+    for (int w = 0; w < 2; ++w) if (m->cube[w][idx].n > 0) jobs.push_back(Job{w, idx});
   for (size_t b0 = 0; b0 < jobs.size(); b0 += 256) {
     const size_t b1 = std::min(jobs.size(), b0 + 256);
-    std::vector<int> hn(b1 - b0);
+    // input count through d_vgout[j] itself (read before the filter overwrites it with the output count)
+    for (size_t j = b0; j < b1; ++j) h->vgn[j - b0] = m->cube[jobs[j].w][jobs[j].idx].n;
+    LIO_CUDA_OK(stats_h2d(S, m->d_vgout, h->vgn, sizeof(int) * (b1 - b0), st));
+    int launches = 0;
     for (size_t j = b0; j < b1; ++j) {
       lio_pm::Cube &c = m->cube[jobs[j].w][jobs[j].idx];
-      if (c.n > m->vg_cap) return LIO_ERR_CAPACITY;
-      // input count through d_vgout[j] itself (read before the filter overwrites it with the output count)
-      hn[j - b0] = c.n;
-    }
-    LIO_CUDA_OK(cudaMemcpyAsync(m->d_vgout, hn.data(), sizeof(int) * hn.size(), cudaMemcpyHostToDevice, st));
-    LIO_CUDA_OK(cudaStreamSynchronize(st));
-    for (size_t j = b0; j < b1; ++j) {
-      lio_pm::Cube &c = m->cube[jobs[j].w][jobs[j].idx];
-      int rc = m->vg.run(c.p, m->d_vgout + (j - b0), c.n, m->leaf[jobs[j].w], m->d_tmp, m->vg_cap, m->d_vgout + (j - b0), nullptr, st, nullptr);
+      int rc = m->vg.run(c.p, m->d_vgout + (j - b0), c.n, m->leaf[jobs[j].w], m->d_tmp, m->vg_cap, m->d_vgout + (j - b0), nullptr, st, &launches);
       if (rc != LIO_OK) return rc;
       LIO_CUDA_OK(cudaMemcpyAsync(c.p, m->d_tmp, sizeof(float4) * c.n, cudaMemcpyDeviceToDevice, st));   // output <= input count
     }
-    LIO_CUDA_OK(cudaMemcpyAsync(hn.data(), m->d_vgout, sizeof(int) * hn.size(), cudaMemcpyDeviceToHost, st));
-    LIO_CUDA_OK(cudaStreamSynchronize(st));
-    for (size_t j = b0; j < b1; ++j) m->cube[jobs[j].w][jobs[j].idx].n = hn[j - b0];
+    S.launches += launches;
+    LIO_CUDA_OK(stats_d2h(S, h->vgout, m->d_vgout, sizeof(int) * (b1 - b0), st));
+    LIO_CUDA_OK(stats_sync(S, st));
+    for (size_t j = b0; j < b1; ++j) m->cube[jobs[j].w][jobs[j].idx].n = h->vgout[j - b0];
   }
   return LIO_OK;
 }
 
-// PointMapping::Process (:765-1052), imu_inited_ == false, num_stack_frames_ == 1.  Clouds: HOST arrays of n x 4 floats.
-extern "C" int lio_pm_process_host(lio_pm *m, const float *corner_last, int nc, const float *surf_last, int ns, const float transform_sum7[7],
-                                   float transform_tobe_mapped7[7], int info3[3]) {
-  if (!m || !transform_sum7 || nc < 0 || ns < 0 || (nc > 0 && !corner_last) || (ns > 0 && !surf_last)) return LIO_ERR_INVALID;
-  if (nc > m->max_points || ns > m->max_points) return LIO_ERR_CAPACITY;
-  LIO_CUDA_OK(cudaSetDevice(m->device));
+// PointMapping::Process (:765-1052), imu_inited_ == false, num_stack_frames_ == 1, on device clouds: src[w] with a device
+// count clamped to n_max[w] on the device.  Shared by the host and device entries.
+static int pm_core(lio_pm *m, const float4 *const src[2], const int *const n_dev[2], const int n_max[2], const float transform_sum7[7],
+                   float transform_tobe_mapped7[7], int info3[3]) {
   cudaStream_t st = m->stream;
-  const float *src[2] = {corner_last, surf_last};
-  const int nin[2] = {nc, ns};
+  CallStats &S = m->stats;
   m->sum = TwistF{transform_sum7[0], transform_sum7[1], transform_sum7[2], transform_sum7[3], transform_sum7[4], transform_sum7[5], transform_sum7[6]};
   m->tobe = twist_mul(m->tobe, twist_mul(twist_inverse(m->bef), m->sum));   // TransformAssociateToMap :753-756
-  int hcnt[4] = {nc, ns, 0, 0};
-  LIO_CUDA_OK(cudaMemcpyAsync(m->d_cnt, hcnt, sizeof(int) * 2, cudaMemcpyHostToDevice, st));
   for (int w = 0; w < 2; ++w) {
-    if (nin[w] == 0) continue;
-    LIO_CUDA_OK(cudaMemcpyAsync(m->d_in[w], src[w], sizeof(float4) * nin[w], cudaMemcpyHostToDevice, st));
-    // to the map frame with the predicted pose, and back (the reference stacks in the map frame first, :782-800, :1013-1016)
-    k_associate<<<(nin[w] + 255) / 256, 256, 0, st>>>(m->d_in[w], m->d_stack[w], m->d_cnt + w, m->tobe, 0);
-    k_associate<<<(nin[w] + 255) / 256, 256, 0, st>>>(m->d_stack[w], m->d_stack[w], m->d_cnt + w, m->tobe, 1);
+    if (n_max[w] == 0) continue;
+    k_associate<<<(n_max[w] + 255) / 256, 256, 0, st>>>(src[w], m->d_stack[w], n_dev[w], n_max[w], m->d_cnt + w, m->tobe);
+    ++S.launches;
   }
-  LIO_CUDA_OK(cudaStreamSynchronize(st));   // hcnt is a stack array
   float z[3];
   {  // point_on_z_axis_ = tobe * (0, 0, 10)
     rotate_host(m->tobe, 0.0f, 0.0f, 10.0f, z[0], z[1], z[2]);
@@ -381,20 +456,22 @@ extern "C" int lio_pm_process_host(lio_pm *m, const float *corner_last, int nc, 
   for (int w = 0; w < 2; ++w) { int rc = pm_from_map(m, valid, w, K[w]); if (rc != LIO_OK) return rc; }
   m->last_from_map[0] = K[0]; m->last_from_map[1] = K[1];
   // down-sample the stacks
-  int n_ds[2] = {0, 0};
+  int launches = 0;
   for (int w = 0; w < 2; ++w) {
-    if (nin[w] == 0) { LIO_CUDA_OK(cudaMemsetAsync(m->d_cnt + 2 + w, 0, sizeof(int), st)); continue; }
-    int rc = m->vg.run(m->d_stack[w], m->d_cnt + w, nin[w], m->leaf[w], m->d_ds[w], m->max_points, m->d_cnt + 2 + w, nullptr, st, nullptr);
+    if (n_max[w] == 0) { LIO_CUDA_OK(cudaMemsetAsync(m->d_cnt + 2 + w, 0, sizeof(int), st)); continue; }
+    int rc = m->vg.run(m->d_stack[w], m->d_cnt + w, n_max[w], m->leaf[w], m->d_ds[w], m->max_points, m->d_cnt + 2 + w, nullptr, st, &launches);
     if (rc != LIO_OK) return rc;
   }
-  LIO_CUDA_OK(cudaMemcpyAsync(hcnt + 2, m->d_cnt + 2, sizeof(int) * 2, cudaMemcpyDeviceToHost, st));
-  LIO_CUDA_OK(cudaStreamSynchronize(st));
-  n_ds[0] = hcnt[2]; n_ds[1] = hcnt[3];
+  S.launches += launches;
+  LIO_CUDA_OK(stats_d2h(S, m->h->n_ds, m->d_cnt + 2, sizeof(int) * 2, st));
+  LIO_CUDA_OK(stats_sync(S, st));
+  const int n_ds[2] = {m->h->n_ds[0], m->h->n_ds[1]};
   // OptimizeTransformTobeMapped against the pulled map
   const bool optimised = !(K[0] <= 10 || K[1] <= 100);
   m->last_iters = 0;
   if (optimised && m->max_iter > 0) {
     if (K[0] > m->stm_cap[0] || K[1] > m->stm_cap[1] || n_ds[0] + n_ds[1] > m->stm_cap[2]) {
+      if (m->stm_cap[0] > 0) ++S.syncs;   // cudaFree of the old workspace synchronises the device
       m->stm.destroy();
       m->stm_cap[0] = std::max(2 * K[0], 1 << 15); m->stm_cap[1] = std::max(2 * K[1], 1 << 16); m->stm_cap[2] = std::max(2 * (n_ds[0] + n_ds[1]), 1 << 15);
       if (m->stm.init(m->stm_cap[0], m->stm_cap[1], m->stm_cap[2]) != 0) { lio_set_last_error(__FILE__, __LINE__, "scan-to-map workspace allocation failed"); return LIO_ERR_CUDA; }
@@ -402,18 +479,63 @@ extern "C" int lio_pm_process_host(lio_pm *m, const float *corner_last, int nc, 
     float tf7[7] = {m->tobe.qx, m->tobe.qy, m->tobe.qz, m->tobe.qw, m->tobe.px, m->tobe.py, m->tobe.pz};
     int rc = scan_to_map_run(m->stm, m->d_map[0], K[0], m->d_map[1], K[1], m->d_ds[0], m->d_cnt + 2, std::max(n_ds[0], 1), m->d_ds[1], m->d_cnt + 3,
                              std::max(n_ds[1], 1), tf7, m->min_match_sq_dis, m->min_plane_dis, m->max_iter, m->delta_r_abort, m->delta_t_abort, 0, nullptr,
-                             &m->last_iters, m->sm, st);
+                             &m->last_iters, m->sm, st, &S);
     if (rc != LIO_OK) return rc;
     m->tobe = TwistF{tf7[0], tf7[1], tf7[2], tf7[3], tf7[4], tf7[5], tf7[6]};
   }
   if (optimised) { m->bef = m->sum; m->aft = m->tobe; }   // TransformUpdate sits behind the optimiser's early return (:327-329, :716)
   int rc = pm_update(m, valid, n_ds);
   if (rc != LIO_OK) return rc;
+  LIO_CUDA_OK(cudaGetLastError());
   if (transform_tobe_mapped7) {
     transform_tobe_mapped7[0] = m->tobe.qx; transform_tobe_mapped7[1] = m->tobe.qy; transform_tobe_mapped7[2] = m->tobe.qz; transform_tobe_mapped7[3] = m->tobe.qw;
     transform_tobe_mapped7[4] = m->tobe.px; transform_tobe_mapped7[5] = m->tobe.py; transform_tobe_mapped7[6] = m->tobe.pz;
   }
   if (info3) { info3[0] = m->last_iters; info3[1] = K[0]; info3[2] = K[1]; }
+  return LIO_OK;
+}
+
+// Host arrays of n x 4 floats: uploaded into the context's buffers, then the same core.
+extern "C" int lio_pm_process_host(lio_pm *m, const float *corner_last, int nc, const float *surf_last, int ns, const float transform_sum7[7],
+                                   float transform_tobe_mapped7[7], int info3[3]) {
+  if (!m || !transform_sum7 || nc < 0 || ns < 0 || (nc > 0 && !corner_last) || (ns > 0 && !surf_last)) return LIO_ERR_INVALID;
+  if (nc > m->max_points || ns > m->max_points) return LIO_ERR_CAPACITY;
+  LIO_CUDA_OK(cudaSetDevice(m->device));
+  cudaStream_t st = m->stream;
+  m->stats.reset();
+  const float *src[2] = {corner_last, surf_last};
+  const int nin[2] = {nc, ns};
+  for (int w = 0; w < 2; ++w) {
+    m->h->cnt_up[w] = nin[w];
+    if (nin[w]) LIO_CUDA_OK(stats_h2d(m->stats, m->d_in[w], src[w], sizeof(float4) * nin[w], st));
+  }
+  LIO_CUDA_OK(stats_h2d(m->stats, m->d_cnt + 4, m->h->cnt_up, sizeof(int) * 2, st));
+  const float4 *const din[2] = {m->d_in[0], m->d_in[1]};
+  const int *const dn[2] = {m->d_cnt + 4, m->d_cnt + 5};
+  return pm_core(m, din, dn, nin, transform_sum7, transform_tobe_mapped7, info3);
+}
+
+extern "C" int lio_pm_process_dev(lio_pm *m, const lio_dev_cloud *corner_last, const lio_dev_cloud *surf_last, const float transform_sum7[7],
+                                  float transform_tobe_mapped7[7], int info3[3]) {
+  if (!m || !transform_sum7 || !corner_last || !surf_last) return LIO_ERR_INVALID;
+  const lio_dev_cloud *c[2] = {corner_last, surf_last};
+  for (int w = 0; w < 2; ++w)
+    if (c[w]->n_max < 0 || (c[w]->n_max > 0 && (!c[w]->xyzi || !c[w]->n_dev))) return LIO_ERR_INVALID;
+  if (corner_last->n_max > m->max_points || surf_last->n_max > m->max_points) {
+    lio_set_last_error(__FILE__, __LINE__, "lio_pm_process_dev: n_max exceeds the max_points given to lio_pm_create");
+    return LIO_ERR_CAPACITY;
+  }
+  LIO_CUDA_OK(cudaSetDevice(m->device));
+  m->stats.reset();
+  const float4 *const src[2] = {reinterpret_cast<const float4 *>(c[0]->xyzi), reinterpret_cast<const float4 *>(c[1]->xyzi)};
+  const int *const dn[2] = {c[0]->n_max > 0 ? c[0]->n_dev : m->d_cnt + 7, c[1]->n_max > 0 ? c[1]->n_dev : m->d_cnt + 7};
+  const int nmax[2] = {c[0]->n_max, c[1]->n_max};
+  return pm_core(m, src, dn, nmax, transform_sum7, transform_tobe_mapped7, info3);
+}
+
+extern "C" int lio_pm_last_stats(lio_pm *m, long long out[4]) {
+  if (!m || !out) return LIO_ERR_INVALID;
+  out[0] = m->stats.launches; out[1] = m->stats.syncs; out[2] = m->stats.h2d; out[3] = m->stats.d2h;
   return LIO_OK;
 }
 

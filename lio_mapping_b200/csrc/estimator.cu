@@ -2498,7 +2498,8 @@ int ScanToMapWork::init(int cap_corner_map, int cap_surf_map, int cap_queries) {
   auto alloc = [](void **p, size_t bytes) { return cudaMalloc(p, bytes ? bytes : 16) == cudaSuccess; };
   if (!(alloc((void **)&fo.pts, sizeof(float4) * cap_feat) && alloc((void **)&fo.coef, sizeof(float4) * cap_feat) &&
         alloc((void **)&fo.src, sizeof(int) * cap_feat) && alloc((void **)&d_n, sizeof(int) * 8) && alloc((void **)&d_tf, sizeof(TransformF)) &&
-        alloc((void **)&d_odom, sizeof(OdomState)) && alloc((void **)&d_partial, sizeof(double) * 32 * 1024) && alloc((void **)&d_z, sizeof(float) * 4)))
+        alloc((void **)&d_odom, sizeof(OdomState)) && alloc((void **)&d_partial, sizeof(double) * 32 * 1024) && alloc((void **)&d_z, sizeof(float) * 4) &&
+        cudaMallocHost((void **)&h_stage, 64) == cudaSuccess))
     return -1;
   fo.cap = cap_feat;
   fo.count = d_n + 4;
@@ -2508,23 +2509,32 @@ int ScanToMapWork::init(int cap_corner_map, int cap_surf_map, int cap_queries) {
 void ScanToMapWork::destroy() {
   void *fr[] = {fo.pts, fo.coef, fo.src, d_n, d_tf, d_odom, d_partial, d_z};
   for (void *q : fr) if (q) cudaFree(q);
+  if (h_stage) cudaFreeHost(h_stage);
   hc.destroy(); hs.destroy(); w.destroy();
-  fo = FeatureOut(); d_n = nullptr; d_tf = nullptr; d_odom = nullptr; d_partial = nullptr; d_z = nullptr;
+  fo = FeatureOut(); d_n = nullptr; d_tf = nullptr; d_odom = nullptr; d_partial = nullptr; d_z = nullptr; h_stage = nullptr;
 }
 
 // Maps and stacks are device arrays; Kc / Ks are known on the host (the caller assembled the maps), the stack sizes are
-// device counts bounded by Mc_max / Ms_max.  tf7 (host, in/out).  No synchronisation before the final read-back.
+// device counts bounded by Mc_max / Ms_max.  tf7 (host, in/out).  The uploads go through the workspace's pinned staging,
+// so the only synchronisation is the final read-back.  stats (optional) accumulates launches, the sync and the copies.
 int scan_to_map_run(ScanToMapWork &W, const float4 *d_cmap, int Kc, const float4 *d_smap, int Ks, const float4 *d_corner, const int *d_nc,
                     int Mc_max, const float4 *d_surf, const int *d_ns, int Ms_max, float *tf7, float min_match_sq_dis, float min_plane_dis,
-                    int max_iter, double delta_r_abort, double delta_t_abort, int variant, int *n_out, int *iters, int sm, cudaStream_t st) {
+                    int max_iter, double delta_r_abort, double delta_t_abort, int variant, int *n_out, int *iters, int sm, cudaStream_t st,
+                    CallStats *stats) {
   if (n_out) *n_out = 0;
   if (iters) *iters = 0;
   if (Kc <= 10 || Ks <= 100 || max_iter == 0) return LIO_OK;  // PointMapping.cc:327-329: nothing to optimise against
   if (Mc_max + Ms_max > W.cap_feat) { lio_set_last_error(__FILE__, __LINE__, "scan-to-map: stacks exceed the feature capacity"); return LIO_ERR_CAPACITY; }
-  const int hn[2] = {Kc, Ks};
-  LIO_CUDA_OK(cudaMemcpyAsync(W.d_n, hn, sizeof(hn), cudaMemcpyHostToDevice, st));
+  CallStats local;
+  CallStats &S = stats ? *stats : local;
+  int *hn = reinterpret_cast<int *>(W.h_stage);              // [0, 8)   Kc, Ks
+  float *hz = reinterpret_cast<float *>(W.h_stage + 16);     // [16, 32) point_on_z_axis_
+  float *htf = reinterpret_cast<float *>(W.h_stage + 32);    // [32, 60) start pose
+  hn[0] = Kc; hn[1] = Ks;
+  std::memcpy(htf, tf7, sizeof(TransformF));
+  LIO_CUDA_OK(stats_h2d(S, W.d_n, hn, 2 * sizeof(int), st));
   LIO_CUDA_OK(cudaMemsetAsync(W.d_n + 4, 0, sizeof(int), st));
-  LIO_CUDA_OK(cudaMemcpyAsync(W.d_tf, tf7, sizeof(TransformF), cudaMemcpyHostToDevice, st));
+  LIO_CUDA_OK(stats_h2d(S, W.d_tf, htf, sizeof(TransformF), st));
   LIO_CUDA_OK(cudaMemsetAsync(W.d_odom, 0, sizeof(OdomState), st));
   {  // point_on_z_axis_ = T0 * (0, 0, 10), fixed for the whole optimisation (PointMapping.cc:803-806); float, no FMA
     const float qx = tf7[0], qy = tf7[1], qz = tf7[2], qw = tf7[3], vx = 0.0f, vy = 0.0f, vz = 10.0f;
@@ -2534,36 +2544,37 @@ int scan_to_map_run(ScanToMapWork &W, const float4 *d_cmap, int Kc, const float4
     volatile float ax = ux2 * qw, ay = uy2 * qw, az = uz2 * qw;
     volatile float rx = vx + ax, ry = vy + ay, rz = vz + az;
     volatile float sx = rx + cx, sy = ry + cy, sz = rz + cz;
-    const float hz[4] = {sx + tf7[4], sy + tf7[5], sz + tf7[6], 0.f};
-    LIO_CUDA_OK(cudaMemcpyAsync(W.d_z, hz, sizeof(hz), cudaMemcpyHostToDevice, st));
-    LIO_CUDA_OK(cudaStreamSynchronize(st));   // hn / hz are stack variables
+    hz[0] = sx + tf7[4]; hz[1] = sy + tf7[5]; hz[2] = sz + tf7[6]; hz[3] = 0.f;
+    LIO_CUDA_OK(stats_h2d(S, W.d_z, hz, 4 * sizeof(float), st));
   }
   const float cell = sqrtf(min_match_sq_dis) * (1.0f + 1.0f / 1024.0f);
-  int rc = W.hc.build(d_cmap, W.d_n, Kc, cell, st, nullptr);
-  if (rc == LIO_OK) rc = W.hs.build(d_smap, W.d_n + 1, Ks, cell, st, nullptr);
+  int launches = 0;
+  int rc = W.hc.build(d_cmap, W.d_n, Kc, cell, st, &launches);
+  if (rc == LIO_OK) rc = W.hs.build(d_smap, W.d_n + 1, Ks, cell, st, &launches);
   const int cap = std::max(1, Mc_max + Ms_max);
   const int nb = std::max(1, std::min(sm, (cap + kOdomThreads - 1) / kOdomThreads));
   for (int it = 0; it < max_iter && rc == LIO_OK; ++it) {
     rc = calculate_features_dev(W.hc, d_cmap, d_corner, d_nc, std::max(Mc_max, 1), W.d_tf, min_match_sq_dis, min_plane_dis, W.fo, 0,
-                                &W.d_odom->done, W.w, st, nullptr, 3, W.d_z);
+                                &W.d_odom->done, W.w, st, &launches, 3, W.d_z);
     if (rc == LIO_OK)
       rc = calculate_features_dev(W.hs, d_smap, d_surf, d_ns, std::max(Ms_max, 1), W.d_tf, min_match_sq_dis, min_plane_dis, W.fo, 1,
-                                  &W.d_odom->done, W.w, st, nullptr, 2, W.d_z);
+                                  &W.d_odom->done, W.w, st, &launches, 2, W.d_z);
     if (rc != LIO_OK) break;
     k_odom_reduce<<<nb, kOdomThreads, 0, st>>>(W.fo.pts, W.fo.coef, W.fo.count, W.d_tf, W.d_odom, W.d_partial, variant == 1 ? 2 : 1);
     k_odom_solve<<<1, 32, 0, st>>>(W.d_odom, W.d_tf, delta_r_abort, delta_t_abort, it, W.fo.count, 50, variant == 1 ? 1 : 0);
+    launches += 2;
   }
+  S.launches += launches;
   if (rc != LIO_OK) return rc;
-  int m = 0;
-  OdomState hs2;
-  cudaError_t ce = cudaMemcpyAsync(&m, W.d_n + 4, sizeof(int), cudaMemcpyDeviceToHost, st);
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(&hs2, W.d_odom, sizeof(OdomState), cudaMemcpyDeviceToHost, st);
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(tf7, W.d_tf, sizeof(TransformF), cudaMemcpyDeviceToHost, st);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(st);
+  int m = 0, it_done = 0;
+  cudaError_t ce = stats_d2h(S, &m, W.d_n + 4, sizeof(int), st);
+  if (ce == cudaSuccess) ce = stats_d2h(S, &it_done, &W.d_odom->iter, sizeof(int), st);
+  if (ce == cudaSuccess) ce = stats_d2h(S, tf7, W.d_tf, sizeof(TransformF), st);
+  if (ce == cudaSuccess) ce = stats_sync(S, st);
   if (ce != cudaSuccess) { lio_set_last_error(__FILE__, __LINE__, cudaGetErrorString(ce)); return LIO_ERR_CUDA; }
   if (m > cap) { lio_set_last_error(__FILE__, __LINE__, "feature buffer overflow"); return LIO_ERR_CAPACITY; }
   if (n_out) *n_out = m;
-  if (iters) *iters = hs2.iter;
+  if (iters) *iters = it_done;
   return LIO_OK;
 }
 

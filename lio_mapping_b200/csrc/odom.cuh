@@ -28,13 +28,15 @@ struct ScanToMapWork {
   OdomState *d_odom = nullptr;
   double *d_partial = nullptr;
   float *d_z = nullptr;
+  unsigned char *h_stage = nullptr;   // pinned: the counts, point_on_z_axis_ and the start pose uploaded by scan_to_map_run
   int cap_feat = 0;
   int init(int cap_corner_map, int cap_surf_map, int cap_queries);
   void destroy();
 };
 int scan_to_map_run(ScanToMapWork &W, const float4 *d_cmap, int Kc, const float4 *d_smap, int Ks, const float4 *d_corner, const int *d_nc,
                     int Mc_max, const float4 *d_surf, const int *d_ns, int Ms_max, float *tf7, float min_match_sq_dis, float min_plane_dis,
-                    int max_iter, double delta_r_abort, double delta_t_abort, int variant, int *n_out, int *iters, int sm, cudaStream_t st);
+                    int max_iter, double delta_r_abort, double delta_t_abort, int variant, int *n_out, int *iters, int sm, cudaStream_t st,
+                    CallStats *stats = nullptr);
 
 // rot.toRotationMatrix() of the (possibly un-normalised) float quaternion
 __device__ __forceinline__ void odom_rotation(const TransformF &tf, float (&R)[9]) {

@@ -63,10 +63,18 @@ __device__ __forceinline__ float4 po_to_start(float4 pi, const TransformF &es, f
   return po;
 }
 
-// PointOdometry::TransformToEnd :261-292, in place
-__global__ void __launch_bounds__(256) po_to_end(float4 *__restrict__ cloud, int n, TransformF es, float time_factor) {
+// PointOdometry::TransformToEnd :261-292, in place, on *n_dev points with transform_es_ from the device.  normalise: the
+// rotation normalised first (transform_es_.rot.normalize() :675, the host's float expression), as the full cloud of
+// PublishResults sees it.
+__global__ void __launch_bounds__(256) po_to_end(float4 *__restrict__ cloud, const int *__restrict__ n_dev, const TransformF *__restrict__ tf_dev,
+                                                 int normalise, float time_factor) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
+  if (i >= *n_dev) return;
+  TransformF es = *tf_dev;
+  if (normalise) {
+    const float n = sqrtf(es.qx * es.qx + es.qy * es.qy + es.qz * es.qz + es.qw * es.qw);
+    es.qx /= n; es.qy /= n; es.qz /= n; es.qw /= n;
+  }
   float4 p = cloud[i];
   const float s = time_factor * (p.w - (float)(int)p.w);
   p.x -= s * es.px; p.y -= s * es.py; p.z -= s * es.pz;
@@ -77,6 +85,27 @@ __global__ void __launch_bounds__(256) po_to_end(float4 *__restrict__ cloud, int
   odom_qmul_vec(cx, cy, cz, cw, p.x, p.y, p.z, ax, ay, az);
   odom_qmul_vec(es.qx, es.qy, es.qz, es.qw, ax, ay, az, bx, by, bz);
   cloud[i] = make_float4(bx + es.px, by + es.py, bz + es.pz, p.w);
+}
+
+// Ingest of the device entry: the five counts read on the device and clamped to their bounds into cnt[0..4], and the
+// clouds that outlive the call (less sharp, less flat, full: blockIdx.y 0..2) copied into the context's buffers.
+struct PoIngest {
+  const float4 *src[3];
+  float4 *dst[3];
+  const int *n_in[5];
+  int n_max[5];
+};
+__global__ void __launch_bounds__(256) po_ingest(PoIngest a, int *__restrict__ cnt) {
+  const int y = blockIdx.y;
+  const int k = y == 0 ? 1 : (y == 1 ? 3 : 4);   // count slot of the copied cloud
+  int n = *a.n_in[k];
+  n = n < 0 ? 0 : (n > a.n_max[k] ? a.n_max[k] : n);
+  if (blockIdx.x == 0 && y == 0 && threadIdx.x < 5) {
+    const int j = threadIdx.x;
+    const int v = *a.n_in[j];
+    cnt[j] = v < 0 ? 0 : (v > a.n_max[j] ? a.n_max[j] : v);
+  }
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) a.dst[y][i] = __ldg(a.src[y] + i);
 }
 
 __device__ __forceinline__ unsigned long long po_min64(unsigned long long a, unsigned long long b) { return a < b ? a : b; }
@@ -95,9 +124,10 @@ __device__ __forceinline__ int po_visit_to_index(unsigned v, int c) { return v <
 // last_surf_cloud_ (3 indices per query).
 template <int KIND>
 __global__ void __launch_bounds__(kPoSearchThreads)
-po_search(const float4 *__restrict__ query, int nq, const float4 *__restrict__ last, int nlast, const TransformF *__restrict__ tf_dev,
-          const OdomState *__restrict__ st, float time_factor, int *__restrict__ idx_out) {
-  if (st->done) return;
+po_search(const float4 *__restrict__ query, const int *__restrict__ nq_dev, const float4 *__restrict__ last, int nlast,
+          const TransformF *__restrict__ tf_dev, const OdomState *__restrict__ st, float time_factor, int *__restrict__ idx_out) {
+  const int nq = *nq_dev;   // the grid covers the bound; CTAs past the count leave at once
+  if (st->done || (int)blockIdx.x * kPoQ >= nq) return;
   __shared__ float4 s_sel[kPoQ];
   __shared__ unsigned long long s_best[kPoSearchThreads / 32][kPoQ];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -190,10 +220,11 @@ po_search(const float4 *__restrict__ query, int nq, const float4 *__restrict__ l
 
 // One iteration of the loop :333-664 after the searches: coefficients, normal equations, solve, update, convergence.
 __global__ void __launch_bounds__(kPoRoundThreads)
-po_round(const float4 *__restrict__ sharp, int ns, const float4 *__restrict__ flat, int nf, const float4 *__restrict__ last_corner,
+po_round(const float4 *__restrict__ sharp, const float4 *__restrict__ flat, const int *__restrict__ counts, const float4 *__restrict__ last_corner,
          const float4 *__restrict__ last_surf, const int *__restrict__ idx_c, const int *__restrict__ idx_s, TransformF *__restrict__ tf_dev,
          OdomState *__restrict__ st, float time_factor, int iter, int *__restrict__ nsel_out) {
   if (st->done) return;
+  const int ns = counts[0], nf = counts[2];   // sharp, flat
   __shared__ double s_red[kPoRoundThreads / 32][28];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const TransformF es = *tf_dev;
@@ -298,6 +329,15 @@ po_round(const float4 *__restrict__ sharp, int ns, const float4 *__restrict__ fl
 
 using namespace lio;
 
+// Pinned staging of one process call: what goes up (start pose, host-path counts) and the single read-back.
+struct PoStage {
+  TransformF tf_up;
+  int cnt_up[5];
+  int cnt[5];      // sharp, less_sharp, flat, less_flat, full as the kernels saw them (clamped)
+  int iter, nsel;
+  TransformF tf;
+};
+
 struct lio_po {
   int device = 0;
   cudaStream_t stream = nullptr;
@@ -308,21 +348,27 @@ struct lio_po {
   long frame_count = 0;
   float4 *d_sharp = nullptr, *d_flat = nullptr, *d_less_sharp = nullptr, *d_less_flat = nullptr, *d_last_corner = nullptr, *d_last_surf = nullptr,
          *d_full = nullptr;
-  int n_sharp = 0, n_flat = 0, n_less_sharp = 0, n_less_flat = 0, n_last_corner = 0, n_last_surf = 0, n_full = 0;
+  int n_sharp = 0, n_flat = 0, n_less_sharp = 0, n_less_flat = 0, n_last_corner = 0, n_last_surf = 0, n_full = 0;   // host copies (read-back)
+  // device counts of the last call: [0] sharp [1] less_sharp (now last_corner) [2] flat [3] less_flat (now last_surf) [4] full;
+  // [7] stays 0 (the count of an absent cloud)
+  int *d_cnt = nullptr;
   int *d_idx_c = nullptr, *d_idx_s = nullptr, *d_nsel = nullptr;
   TransformF *d_tf = nullptr;
   OdomState *d_odom = nullptr;
+  PoStage *h_stage = nullptr;
   TwistF es, sum;
   int published = 0;
   int launches = 0;
+  CallStats stats;
 };
 
 extern "C" int lio_po_destroy(lio_po *p) {
   if (!p) return LIO_OK;
   cudaSetDevice(p->device);
-  void *fr[] = {p->d_sharp, p->d_flat, p->d_less_sharp, p->d_less_flat, p->d_last_corner, p->d_last_surf, p->d_full, p->d_idx_c, p->d_idx_s,
-                p->d_nsel, p->d_tf, p->d_odom};
+  void *fr[] = {p->d_sharp, p->d_flat, p->d_less_sharp, p->d_less_flat, p->d_last_corner, p->d_last_surf, p->d_full, p->d_cnt, p->d_idx_c,
+                p->d_idx_s, p->d_nsel, p->d_tf, p->d_odom};
   for (void *q : fr) if (q) cudaFree(q);
+  if (p->h_stage) cudaFreeHost(p->h_stage);
   delete p;
   return LIO_OK;
 }
@@ -341,11 +387,13 @@ extern "C" int lio_po_create(float scan_period, int io_ratio, int num_max_iterat
   float4 **clouds[] = {&p->d_sharp, &p->d_flat, &p->d_less_sharp, &p->d_less_flat, &p->d_last_corner, &p->d_last_surf};
   for (float4 **c : clouds) ok = ok && cudaMalloc(c, sizeof(float4) * max_feature_points) == cudaSuccess;
   ok = ok && cudaMalloc(&p->d_full, sizeof(float4) * max_full_points) == cudaSuccess;
+  ok = ok && cudaMalloc(&p->d_cnt, sizeof(int) * 8) == cudaSuccess && cudaMemset(p->d_cnt, 0, sizeof(int) * 8) == cudaSuccess;
   ok = ok && cudaMalloc(&p->d_idx_c, sizeof(int) * 2 * max_feature_points) == cudaSuccess;
   ok = ok && cudaMalloc(&p->d_idx_s, sizeof(int) * 3 * max_feature_points) == cudaSuccess;
   ok = ok && cudaMalloc(&p->d_nsel, sizeof(int)) == cudaSuccess;
   ok = ok && cudaMalloc(&p->d_tf, sizeof(TransformF)) == cudaSuccess;
   ok = ok && cudaMalloc(&p->d_odom, sizeof(OdomState)) == cudaSuccess;
+  ok = ok && cudaMallocHost(&p->h_stage, sizeof(PoStage)) == cudaSuccess;
   if (!ok) { lio_set_last_error(__FILE__, __LINE__, "lio_po_create: device allocation failed"); lio_po_destroy(p); return LIO_ERR_CUDA; }
   *out = p;
   return LIO_OK;
@@ -359,6 +407,84 @@ extern "C" int lio_po_set_enable_odom(lio_po *p, int enable) {   // the /enable_
 
 static void po_store(const TwistF &t, float *o) { o[0] = t.qx; o[1] = t.qy; o[2] = t.qz; o[3] = t.qw; o[4] = t.px; o[5] = t.py; o[6] = t.pz; }
 
+// Process + PublishResults (:294-766) once the sweep is in place: less sharp / less flat / full in the context's buffers,
+// the five clamped counts in d_cnt[0..4], sharp / flat at `sharp` / `flat` (the caller's buffers or the context's).  mx_*
+// bound the counts and size the grids.  One synchronisation: the read-back of transform_es_, the iteration and match
+// counts and the five counts, from which the host learns the sizes of the new "last" clouds (the :324 gate of the next call).
+static int po_core(lio_po *p, const float4 *sharp, int mx_sharp, const float4 *flat, int mx_flat, int mx_less_sharp, int mx_less_flat, int mx_full,
+                   float transform_sum7[7], float transform_es7[7], int info4[4]) {
+  cudaStream_t st = p->stream;
+  CallStats &S = p->stats;
+  PoStage *h = p->h_stage;
+  const float tfac = p->time_factor;
+  const bool first = !p->system_inited;   // :302-310: the first sweep only becomes the last clouds
+  bool solved = false;
+  p->published = 0;
+  auto to_end = [&](float4 *cloud, const int *n_dev, int n_max, int normalise) {
+    if (n_max > 0) { po_to_end<<<(n_max + 255) / 256, 256, 0, st>>>(cloud, n_dev, p->d_tf, normalise, tfac); ++p->launches; }
+  };
+  if (first) {
+    p->system_inited = true;
+  } else {
+    ++p->frame_count;
+    if (p->enable_odom) {
+      h->tf_up = TransformF{p->es.qx, p->es.qy, p->es.qz, p->es.qw, p->es.px, p->es.py, p->es.pz};
+      LIO_CUDA_OK(stats_h2d(S, p->d_tf, &h->tf_up, sizeof(TransformF), st));
+      if (p->n_last_corner > 10 && p->n_last_surf > 100) {   // :324
+        LIO_CUDA_OK(cudaMemsetAsync(p->d_odom, 0, sizeof(OdomState), st));
+        LIO_CUDA_OK(cudaMemsetAsync(p->d_nsel, 0, sizeof(int), st));
+        for (int it = 0; it < p->max_iter; ++it) {
+          if (it % 5 == 0) {
+            if (mx_sharp) { po_search<0><<<(mx_sharp + kPoQ - 1) / kPoQ, kPoSearchThreads, 0, st>>>(sharp, p->d_cnt + 0, p->d_last_corner, p->n_last_corner, p->d_tf, p->d_odom, tfac, p->d_idx_c); ++p->launches; }
+            if (mx_flat) { po_search<1><<<(mx_flat + kPoQ - 1) / kPoQ, kPoSearchThreads, 0, st>>>(flat, p->d_cnt + 2, p->d_last_surf, p->n_last_surf, p->d_tf, p->d_odom, tfac, p->d_idx_s); ++p->launches; }
+          }
+          po_round<<<1, kPoRoundThreads, 0, st>>>(sharp, flat, p->d_cnt, p->d_last_corner, p->d_last_surf, p->d_idx_c, p->d_idx_s, p->d_tf, p->d_odom, tfac,
+                                                 it, p->d_nsel);
+          ++p->launches;
+        }
+        solved = true;
+      }
+      // de-skew of the clouds that become the last ones (:673-674) with the unnormalised transform_es_
+      to_end(p->d_less_sharp, p->d_cnt + 1, mx_less_sharp, 0);
+      to_end(p->d_less_flat, p->d_cnt + 3, mx_less_flat, 0);
+    }
+    if (p->io_ratio < 2 || p->frame_count % p->io_ratio == 1) {   // PublishResults :726-765
+      if (p->enable_odom) to_end(p->d_full, p->d_cnt + 4, mx_full, 1);
+      p->published = 1;
+    }
+  }
+  LIO_CUDA_OK(cudaGetLastError());
+  LIO_CUDA_OK(stats_d2h(S, h->cnt, p->d_cnt, sizeof(h->cnt), st));
+  if (solved) {
+    LIO_CUDA_OK(stats_d2h(S, &h->tf, p->d_tf, sizeof(TransformF), st));
+    LIO_CUDA_OK(stats_d2h(S, &h->iter, &p->d_odom->iter, sizeof(int), st));
+    LIO_CUDA_OK(stats_d2h(S, &h->nsel, p->d_nsel, sizeof(int), st));
+  }
+  LIO_CUDA_OK(stats_sync(S, st));
+  LIO_CUDA_OK(cudaGetLastError());
+  S.launches = p->launches;
+  p->n_sharp = h->cnt[0]; p->n_less_sharp = h->cnt[1]; p->n_flat = h->cnt[2]; p->n_less_flat = h->cnt[3]; p->n_full = h->cnt[4];
+  int iters = 0, nsel = 0;
+  if (solved) {
+    p->es = TwistF{h->tf.qx, h->tf.qy, h->tf.qz, h->tf.qw, h->tf.px, h->tf.py, h->tf.pz};
+    iters = h->iter; nsel = h->nsel;
+  }
+  if (!first && p->enable_odom) {
+    p->sum = twist_mul(p->sum, twist_inverse(p->es));   // transform_sum_ = transform_sum_ * transform_es_.inverse()  :667-669
+    const float n = std::sqrt(p->es.qx * p->es.qx + p->es.qy * p->es.qy + p->es.qz * p->es.qz + p->es.qw * p->es.qw);   // :675
+    p->es.qx /= n; p->es.qy /= n; p->es.qz /= n; p->es.qw /= n;
+  }
+  // corner_points_less_sharp_.swap(last_corner_cloud_), surf_points_less_flat_.swap(last_surf_cloud_); the device counts stay in
+  // d_cnt[1] / d_cnt[3]
+  std::swap(p->d_less_sharp, p->d_last_corner); std::swap(p->n_less_sharp, p->n_last_corner);
+  std::swap(p->d_less_flat, p->d_last_surf); std::swap(p->n_less_flat, p->n_last_surf);
+  if (transform_sum7) po_store(p->sum, transform_sum7);
+  if (transform_es7) po_store(p->es, transform_es7);
+  if (info4) { info4[0] = iters; info4[1] = p->published; info4[2] = (int)p->frame_count; info4[3] = nsel; }
+  return LIO_OK;
+}
+
+// Host arrays: uploaded into the context's buffers, then the same core.
 extern "C" int lio_po_process_host(lio_po *p, const float *sharp, int n_sharp, const float *less_sharp, int n_less_sharp, const float *flat,
                                    int n_flat, const float *less_flat, int n_less_flat, const float *full, int n_full, float transform_sum7[7],
                                    float transform_es7[7], int info4[4]) {
@@ -371,74 +497,65 @@ extern "C" int lio_po_process_host(lio_po *p, const float *sharp, int n_sharp, c
   }
   LIO_CUDA_OK(cudaSetDevice(p->device));
   cudaStream_t st = p->stream;
+  p->stats.reset(); p->launches = 0;
   const float *src[5] = {sharp, less_sharp, flat, less_flat, full};
   float4 *dst[5] = {p->d_sharp, p->d_less_sharp, p->d_flat, p->d_less_flat, p->d_full};
   const int cnt[5] = {n_sharp, n_less_sharp, n_flat, n_less_flat, n_full};
+  for (int k = 0; k < 5; ++k) {
+    if (cnt[k]) LIO_CUDA_OK(stats_h2d(p->stats, dst[k], src[k], sizeof(float4) * cnt[k], st));
+    p->h_stage->cnt_up[k] = cnt[k];
+  }
+  LIO_CUDA_OK(stats_h2d(p->stats, p->d_cnt, p->h_stage->cnt_up, sizeof(p->h_stage->cnt_up), st));
+  return po_core(p, p->d_sharp, n_sharp, p->d_flat, n_flat, n_less_sharp, n_less_flat, n_full, transform_sum7, transform_es7, info4);
+}
+
+// Device clouds: the counts are clamped on the device and the clouds that outlive the call are copied in (one kernel),
+// sharp / flat are read where they are.
+extern "C" int lio_po_process_dev(lio_po *p, const lio_dev_cloud clouds[5], float transform_sum7[7], float transform_es7[7], int info4[4]) {
+  if (!p || !clouds) return LIO_ERR_INVALID;
   for (int k = 0; k < 5; ++k)
-    if (cnt[k]) LIO_CUDA_OK(cudaMemcpyAsync(dst[k], src[k], sizeof(float4) * cnt[k], cudaMemcpyHostToDevice, st));
-  p->n_sharp = n_sharp; p->n_less_sharp = n_less_sharp; p->n_flat = n_flat; p->n_less_flat = n_less_flat; p->n_full = n_full;
-  p->published = 0; p->launches = 0;
-  int iters = 0, nsel = 0;
-  auto finish = [&]() {
-    if (transform_sum7) po_store(p->sum, transform_sum7);
-    if (transform_es7) po_store(p->es, transform_es7);
-    if (info4) { info4[0] = iters; info4[1] = p->published; info4[2] = (int)p->frame_count; info4[3] = nsel; }
-    return LIO_OK;
-  };
-  auto swap_in = [&]() {   // corner_points_less_sharp_.swap(last_corner_cloud_), surf_points_less_flat_.swap(last_surf_cloud_)
-    std::swap(p->d_less_sharp, p->d_last_corner); std::swap(p->n_less_sharp, p->n_last_corner);
-    std::swap(p->d_less_flat, p->d_last_surf); std::swap(p->n_less_flat, p->n_last_surf);
-  };
-  if (!p->system_inited) {   // :302-310
-    swap_in();
-    p->system_inited = true;
-    LIO_CUDA_OK(cudaStreamSynchronize(st));
-    return finish();
-  }
-  ++p->frame_count;
-  const float tfac = p->time_factor;
-  auto to_end = [&](float4 *cloud, int n) {
-    if (n > 0) { po_to_end<<<(n + 255) / 256, 256, 0, st>>>(cloud, n, TransformF{p->es.qx, p->es.qy, p->es.qz, p->es.qw, p->es.px, p->es.py, p->es.pz}, tfac); ++p->launches; }
-  };
-  if (p->enable_odom) {
-    if (p->n_last_corner > 10 && p->n_last_surf > 100) {   // :324
-      const TransformF tf0{p->es.qx, p->es.qy, p->es.qz, p->es.qw, p->es.px, p->es.py, p->es.pz};
-      LIO_CUDA_OK(cudaMemcpyAsync(p->d_tf, &tf0, sizeof(tf0), cudaMemcpyHostToDevice, st));
-      LIO_CUDA_OK(cudaMemsetAsync(p->d_odom, 0, sizeof(OdomState), st));
-      LIO_CUDA_OK(cudaMemsetAsync(p->d_nsel, 0, sizeof(int), st));
-      for (int it = 0; it < p->max_iter; ++it) {
-        if (it % 5 == 0) {
-          if (n_sharp) { po_search<0><<<(n_sharp + kPoQ - 1) / kPoQ, kPoSearchThreads, 0, st>>>(p->d_sharp, n_sharp, p->d_last_corner, p->n_last_corner, p->d_tf, p->d_odom, tfac, p->d_idx_c); ++p->launches; }
-          if (n_flat) { po_search<1><<<(n_flat + kPoQ - 1) / kPoQ, kPoSearchThreads, 0, st>>>(p->d_flat, n_flat, p->d_last_surf, p->n_last_surf, p->d_tf, p->d_odom, tfac, p->d_idx_s); ++p->launches; }
-        }
-        po_round<<<1, kPoRoundThreads, 0, st>>>(p->d_sharp, n_sharp, p->d_flat, n_flat, p->d_last_corner, p->d_last_surf, p->d_idx_c, p->d_idx_s, p->d_tf,
-                                               p->d_odom, tfac, it, p->d_nsel);
-        ++p->launches;
-      }
-      TransformF tf1;
-      OdomState os;
-      LIO_CUDA_OK(cudaMemcpyAsync(&tf1, p->d_tf, sizeof(tf1), cudaMemcpyDeviceToHost, st));
-      LIO_CUDA_OK(cudaMemcpyAsync(&os, p->d_odom, sizeof(os), cudaMemcpyDeviceToHost, st));
-      LIO_CUDA_OK(cudaMemcpyAsync(&nsel, p->d_nsel, sizeof(int), cudaMemcpyDeviceToHost, st));
-      LIO_CUDA_OK(cudaStreamSynchronize(st));
-      LIO_CUDA_OK(cudaGetLastError());
-      p->es = TwistF{tf1.qx, tf1.qy, tf1.qz, tf1.qw, tf1.px, tf1.py, tf1.pz};
-      iters = os.iter;
+    if (clouds[k].n_max < 0 || (clouds[k].n_max > 0 && (!clouds[k].xyzi || !clouds[k].n_dev))) return LIO_ERR_INVALID;
+  for (int k = 0; k < 5; ++k)
+    if (clouds[k].n_max > (k == 4 ? p->cap_full : p->cap_feat)) {
+      lio_set_last_error(__FILE__, __LINE__, "lio_po_process_dev: n_max exceeds the capacity given to lio_po_create");
+      return LIO_ERR_CAPACITY;
     }
-    p->sum = twist_mul(p->sum, twist_inverse(p->es));   // transform_sum_ = transform_sum_ * transform_es_.inverse()  :667-669
-    to_end(p->d_less_sharp, p->n_less_sharp);
-    to_end(p->d_less_flat, p->n_less_flat);
-    const float n = std::sqrt(p->es.qx * p->es.qx + p->es.qy * p->es.qy + p->es.qz * p->es.qz + p->es.qw * p->es.qw);   // transform_es_.rot.normalize() :675
-    p->es.qx /= n; p->es.qy /= n; p->es.qz /= n; p->es.qw /= n;
+  LIO_CUDA_OK(cudaSetDevice(p->device));
+  cudaStream_t st = p->stream;
+  p->stats.reset(); p->launches = 0;
+  PoIngest a;
+  const int copied[3] = {1, 3, 4};
+  float4 *dst[3] = {p->d_less_sharp, p->d_less_flat, p->d_full};
+  int mx = 0;
+  for (int y = 0; y < 3; ++y) {
+    a.src[y] = reinterpret_cast<const float4 *>(clouds[copied[y]].xyzi);
+    a.dst[y] = dst[y];
+    mx = std::max(mx, clouds[copied[y]].n_max);
   }
-  swap_in();
-  if (p->io_ratio < 2 || p->frame_count % p->io_ratio == 1) {   // PublishResults :726-765
-    if (p->enable_odom) to_end(p->d_full, p->n_full);
-    p->published = 1;
+  for (int k = 0; k < 5; ++k) {
+    a.n_in[k] = clouds[k].n_max > 0 ? clouds[k].n_dev : p->d_cnt + 7;
+    a.n_max[k] = clouds[k].n_max;
   }
-  LIO_CUDA_OK(cudaStreamSynchronize(st));
-  LIO_CUDA_OK(cudaGetLastError());
-  return finish();
+  po_ingest<<<dim3(std::max(1, std::min((mx + 255) / 256, 4 * 148)), 3), 256, 0, st>>>(a, p->d_cnt);
+  ++p->launches;
+  return po_core(p, reinterpret_cast<const float4 *>(clouds[0].xyzi), clouds[0].n_max, reinterpret_cast<const float4 *>(clouds[2].xyzi),
+                 clouds[2].n_max, clouds[1].n_max, clouds[3].n_max, clouds[4].n_max, transform_sum7, transform_es7, info4);
+}
+
+extern "C" int lio_po_cloud_dev(lio_po *p, int which, const float **xyzi, const int **n_dev) {
+  if (!p || !xyzi || !n_dev) return LIO_ERR_INVALID;
+  switch (which) {
+    case 0: *xyzi = reinterpret_cast<const float *>(p->d_last_corner); *n_dev = p->d_cnt + 1; return LIO_OK;
+    case 1: *xyzi = reinterpret_cast<const float *>(p->d_last_surf); *n_dev = p->d_cnt + 3; return LIO_OK;
+    case 2: *xyzi = reinterpret_cast<const float *>(p->d_full); *n_dev = p->d_cnt + 4; return LIO_OK;
+    default: return LIO_ERR_INVALID;
+  }
+}
+
+extern "C" int lio_po_last_stats(lio_po *p, long long out[4]) {
+  if (!p || !out) return LIO_ERR_INVALID;
+  out[0] = p->stats.launches; out[1] = p->stats.syncs; out[2] = p->stats.h2d; out[3] = p->stats.d2h;
+  return LIO_OK;
 }
 
 static int po_cloud(lio_po *p, int which, const float4 **d, int *n) {

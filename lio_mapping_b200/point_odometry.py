@@ -18,6 +18,7 @@ class PointOdometry:
     def __init__(self, scan_period: float = 0.1, io_ratio: int = 2, num_max_iterations: int = 25, max_feature_points: int = 1 << 17,
                  max_full_points: int = 1 << 20, device: int = 0, stream: int = 0):
         _lib.require_device()
+        self.max_feature_points, self.max_full_points = int(max_feature_points), int(max_full_points)
         self.h = C.c_void_p()
         _lib.check(_lib.lib().lio_po_create(scan_period, int(io_ratio), int(num_max_iterations), int(max_feature_points), int(max_full_points),
                                             device, C.c_void_p(stream), C.byref(self.h)), "lio_po_create")
@@ -46,6 +47,35 @@ class PointOdometry:
         ts = np.zeros(7, np.float32); te = np.zeros(7, np.float32); info = np.zeros(4, np.int32)
         _lib.check(_lib.lib().lio_po_process_host(self.h, *args, ts, te, info), "lio_po_process_host")
         return ts, te, dict(iterations=int(info[0]), published=int(info[1]), frame_count=int(info[2]), matches=int(info[3]))
+
+    def process_device(self, pp, n_max=None):
+        """Process on the five stage-A clouds of `pp` (a PointProcessor) where they lie on the device, with their device counts:
+        no host copy of a cloud.  n_max (optional, 5 ints) bounds the counts (a larger device count is clamped to it); default:
+        pp.output_bounds() capped at this context's capacities.  Returns what Process returns.  The clouds that outlive the
+        call are copied into this context, so `pp` may process the next sweep right away."""
+        L = _lib.lib()
+        names = ("corner_points_sharp", "corner_points_less_sharp", "surface_points_flat", "surface_points_less_flat", "laser_scans")
+        if n_max is None:
+            b = pp.output_bounds()
+            n_max = [min(b[k], self.max_feature_points) for k in names[:4]] + [min(b["laser_scans"], self.max_full_points)]
+        clouds = (_lib.DevCloud * 5)()
+        for k, name in enumerate(names):
+            clouds[k] = _lib.DevCloud(pp.cloud_dev(name), pp.count_dev(name), int(n_max[k]))
+        ts = np.zeros(7, np.float32); te = np.zeros(7, np.float32); info = np.zeros(4, np.int32)
+        _lib.check(L.lio_po_process_dev(self.h, clouds, ts, te, info), "lio_po_process_dev")
+        return ts, te, dict(iterations=int(info[0]), published=int(info[1]), frame_count=int(info[2]), matches=int(info[3]))
+
+    def cloud_dev(self, which: str):
+        """(device pointer, device count pointer) of last_corner / last_surf / full; valid until the next process call."""
+        p, n = C.c_void_p(), C.c_void_p()
+        _lib.check(_lib.lib().lio_po_cloud_dev(self.h, _WHICH[which], C.byref(p), C.byref(n)), "lio_po_cloud_dev")
+        return p.value, n.value
+
+    def stats(self) -> dict:
+        """What the last process call cost the host."""
+        out = np.zeros(4, np.int64)
+        _lib.check(_lib.lib().lio_po_last_stats(self.h, out), "lio_po_last_stats")
+        return dict(launches=int(out[0]), syncs=int(out[1]), h2d_bytes=int(out[2]), d2h_bytes=int(out[3]))
 
     def cloud(self, which: str):
         w = _WHICH[which]

@@ -34,6 +34,7 @@ class PointProcessor:
         self._h = C.c_void_p()
         _lib.check(L.lio_pp_create(C.byref(cfg), max_points, device, C.c_void_p(stream), C.byref(self._h)), "lio_pp_create")
         self._cloud = None
+        self.last_input_size = 0
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h:
@@ -55,6 +56,7 @@ class PointProcessor:
         if self._cloud is None:
             raise _lib.LioError("SetInputCloud first")
         _lib.check(_lib.lib().lio_pp_process_host(self._h, self._cloud, self._cloud.shape[0]), "lio_pp_process_host")
+        self.last_input_size = self._cloud.shape[0]
 
     def ProcessWithRingField(self, rings):
         """PointToRing for PointXYZIR input (ring index per point, PointProcessor.cc:428-536) + ExtractFeaturePoints."""
@@ -64,10 +66,21 @@ class PointProcessor:
         if r.shape[0] != self._cloud.shape[0]:
             raise ValueError("one ring index per point")
         _lib.check(_lib.lib().lio_pp_process_host_ring(self._h, self._cloud, r, self._cloud.shape[0]), "lio_pp_process_host_ring")
+        self.last_input_size = self._cloud.shape[0]
 
     def process_device(self, dev_ptr: int, n: int):
         """Device-resident input (float4 array); asynchronous on the processor's stream."""
         _lib.check(_lib.lib().lio_pp_process_dev(self._h, C.c_void_p(dev_ptr), n), "lio_pp_process_dev")
+        self.last_input_size = int(n)
+
+    def output_bounds(self) -> dict:
+        """Upper bounds of the feature cloud sizes of the last process call, known without reading the counts back: at most
+        max_corner_sharp / max_corner_less_sharp / max_surf_flat points per ring and subregion (ExtractFeaturePoints),
+        and never more points than the sweep had."""
+        c, n = self.cfg, self.last_input_size
+        rs = c.num_rings * c.num_scan_subregions
+        return {"corner_points_sharp": min(n, rs * c.max_corner_sharp), "corner_points_less_sharp": min(n, rs * c.max_corner_less_sharp),
+                "surface_points_flat": min(n, rs * c.max_surf_flat), "surface_points_less_flat": n, "laser_scans": n}
 
     # -- results ------------------------------------------------------------------------------
     def sizes(self) -> dict:
@@ -86,6 +99,12 @@ class PointProcessor:
     def cloud_dev(self, name: str) -> int:
         p = C.c_void_p()
         _lib.check(_lib.lib().lio_pp_cloud_dev(self._h, CLOUDS[name], C.byref(p)), "lio_pp_cloud_dev")
+        return p.value
+
+    def count_dev(self, name: str) -> int:
+        """Device pointer of the point count of one output cloud (lio_pp_cloud_count_dev), to chain stage A on the device."""
+        p = C.c_void_p()
+        _lib.check(_lib.lib().lio_pp_cloud_count_dev(self._h, CLOUDS[name], C.byref(p)), "lio_pp_cloud_count_dev")
         return p.value
 
     def index(self, name: str) -> np.ndarray:
